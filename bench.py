@@ -20,8 +20,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
-for p in (ROOT, os.path.join(ROOT, "gaussian-mesh-splatting_b200"), os.path.join(ROOT, "tests"), os.path.join(ROOT, "baseline"),
-          os.path.join(ROOT, "baseline", "refstyle")):
+for p in (ROOT, os.path.join(ROOT, "gaussian-mesh-splatting_b200"), os.path.join(ROOT, "tests"), os.path.join(ROOT, "baseline", "refstyle")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
@@ -124,6 +123,26 @@ def flat_scene(seed=0):
     g = scenes.flat_gaussians(P, seed=seed)
     cam = scenes.look_at_camera((4.03 * math.cos(0.5), 4.03 * math.sin(0.5), 1.2), (0, 0, 0), W, H)
     return g, cam
+
+
+DUMP_MAX_ROWS = 65536            # larger outputs are dumped as a fixed, seeded sample of their rows
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each output of the last timed step as <out_dir>/<name>.npy (float32, or float64 for float64
+    tensors), so that two builds run with the same arguments can be compared array by array.  An array with more than
+    DUMP_MAX_ROWS rows is reduced to the same rows every run: a sorted sample drawn with a fixed seed from its row count."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else np.asarray(t)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32).reshape(a.shape or (1,))
+        if a.shape[0] > DUMP_MAX_ROWS:
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], DUMP_MAX_ROWS, replace=False))]
+        total += a.nbytes
+        assert total <= DUMP_MAX_BYTES, f"--dump-outputs: more than {DUMP_MAX_BYTES} bytes"
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
 
 
 class ClockSampler(threading.Thread):
@@ -317,7 +336,7 @@ def run_render_animated(args, params, cams, dims, dev, world, rank, local):
                 sink.write(img, os.path.join(args.save_images, f"{lo + (i % per):05d}.{args.image_format}"))
             return img
 
-    K_, W_ = min(args.steps, per), max(args.warmup, 3)
+    K_, W_ = args.steps, max(args.warmup, 3)
     for i in range(max(W_, 2 * len(cams_dev))):
         frame(i)
     if world > 1:
@@ -328,7 +347,7 @@ def run_render_animated(args, params, cams, dims, dev, world, rank, local):
     t_wall = time.perf_counter()
     e0.record()
     for i in range(K_):
-        frame(W_ + i)
+        img = frame(W_ + i)
     e1.record()
     if world > 1:
         dist.barrier()
@@ -340,6 +359,8 @@ def run_render_animated(args, params, cams, dims, dev, world, rank, local):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     launches = _lib.launch_count(reset=True)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image": img})
     if rank == 0:
         ms_step = float(ms.item()) / K_
         cfg = base_config(args.workload)
@@ -391,10 +412,12 @@ def run_flat(args, dev):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for s in range(K_):
-        step(s)
+        loss = step(s)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / K_
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(loss=loss, **{f"grad_{k}": v.grad for k, v in t.items()}))
     line = {"metric": METRIC[args.workload], "value": 1000.0 / ms, "unit": "frames/s", "n_gpus": 1, "steps": K_, "warmup": W_,
             "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": base_config(args.workload), "gpu_launches": int(_lib.launch_count(reset=True)),
@@ -411,9 +434,7 @@ def run_comparators(model, cams_dev, gts, bg, dims, dev, n_frames=12):
     """SURVEY.md 8(d) 'how the reference's paths are timed beside it', on the same GPU, same process, same tensors:
     (1) rasterizer-only (R2-R9) fwd+bwd: product vs the ref-style stand-in (baseline/refstyle: Appendix A with the stock
         work decomposition -- NOT the stock binary, whose source is absent);
-    (2) expansion fwd+bwd: the reference's own PyTorch code (GaussianMeshModel.update_alpha / prepare_scaling_rot + getters,
-        from the baseline/_ref snapshot) vs the fused kernels;
-    (3) the reference's frame (train.py:100-108: its render(), its expansion, its utils/loss_utils) on the stand-in."""
+    (2) the image sink vs torchvision.utils.save_image."""
     out = {"label": "ref-style = labelled stand-in for the absent stock diff-gaussian-rasterization (SURVEY Appendix A, stock "
                     "decomposition: CTA/tile, thread/pixel, per-pixel atomics, 64-bit cub sort, host sync); not the stock binary"}
     F, K, W, H = dims
@@ -463,77 +484,7 @@ def run_comparators(model, cams_dev, gts, bg, dims, dev, n_frames=12):
     except Exception as e:  # pragma: no cover
         out["rasterizer_error"] = repr(e)
 
-    try:
-        import ref_snapshot
-        import diff_gaussian_rasterization as ours
-        if not ref_snapshot.import_reference(ours):
-            raise RuntimeError("baseline/_ref snapshot absent")
-        from games.mesh_splatting.scene.gaussian_mesh_model import GaussianMeshModel
-        from gms_b200 import expansion
-        rm = GaussianMeshModel(3)
-        rm.vertices = torch.nn.Parameter(model.vertices.detach().clone())
-        rm.faces = model.faces
-        rm._alpha = torch.nn.Parameter(model._alpha.detach().clone())
-        rm._scale = torch.nn.Parameter(model._scale.detach().clone())
-        P = F * K
-        gen = torch.Generator(device=dev).manual_seed(1)
-        wx, ws, wr = (torch.randn(P, k, device=dev, generator=gen) for k in (3, 3, 4))
-
-        def ref_expand(i):
-            for t in (rm.vertices, rm._alpha, rm._scale):
-                t.grad = None
-            rm.update_alpha(); rm.prepare_scaling_rot()
-            ((rm.get_xyz * wx).sum() + (rm.get_scaling * ws).sum() + (rm.get_rotation * wr).sum()).backward()
-
-        def our_expand(i):
-            x, s, r, _, _ = expansion.expand(model.vertices, model.faces, model._alpha, model._scale, model.eps_s0, True)
-            torch.autograd.grad([x, s, r], [model.vertices, model._alpha, model._scale], [wx, ws, wr])
-
-        ms_r, ms_o = timeit(ref_expand), timeit(our_expand)
-        out["expansion_fwd_bwd_ms"] = {"ours": ms_o, "reference_pytorch": ms_r,
-                                       "reference_code": "games/mesh_splatting/scene/gaussian_mesh_model.py:86-169 + utils/general_utils.py:43-96 "
-                                                         "+ scene/gaussian_model.py:95-101, unmodified, from the baseline/_ref snapshot"}
-        out["vs_reference_expansion"] = ms_r / ms_o
-
-        # (3) the reference's own frame on the stand-in rasterizer
-        import types
-        import refstyle
-        sys.modules["diff_gaussian_rasterization"] = refstyle_module = types.ModuleType("diff_gaussian_rasterization")
-        refstyle_module.GaussianRasterizationSettings = ours.GaussianRasterizationSettings
-        refstyle_module.GaussianRasterizer = refstyle.GaussianRasterizer
-        import importlib
-        import renderer.gaussian_renderer as rgr
-        rgr = importlib.reload(rgr)
-        from scene.cameras import MiniCam
-        from utils.loss_utils import l1_loss, ssim
-        rm._features_dc = torch.nn.Parameter(model._features_dc.detach().clone().contiguous())
-        rm._features_rest = torch.nn.Parameter(model._features_rest.detach().clone().contiguous())
-        rm._opacity = torch.nn.Parameter(model._opacity.detach().clone())
-        rm.active_sh_degree = 3
-        pipe = types.SimpleNamespace(debug=False, antialiasing=False, compute_cov3D_python=False, convert_SHs_python=False)
-        from gms_b200 import scenes
-        minicams = [MiniCam(W, H, c.FoVy, c.FoVx, scenes.ZNEAR, scenes.ZFAR, c.world_view_transform, c.full_proj_transform) for c in cams_dev]
-        plist = [rm.vertices, rm._alpha, rm._scale, rm._features_dc, rm._features_rest, rm._opacity]
-
-        def ref_frame(i):
-            for t in plist:
-                t.grad = None
-            rm.update_alpha(); rm.prepare_scaling_rot()                          # train.py:154-157
-            image = rgr.render(minicams[i % len(minicams)], rm, pipe, bg)["render"]   # train.py:100-101
-            gt = gts[i % len(gts)]
-            loss = (1.0 - 0.2) * l1_loss(image, gt) + 0.2 * (1.0 - ssim(image, gt))   # train.py:105-107
-            loss.backward()                                                       # train.py:108
-
-        ms_f = timeit(ref_frame, n=max(4, n_frames // 2), warm=2)
-        out["reference_frame_on_refstyle"] = {"ms": ms_f, "frames_per_s": 1000.0 / ms_f,
-                                              "what": "the reference's render() + its PyTorch expansion + its ATen L1/SSIM + autograd "
-                                                      "(train.py:100-108,154-157), rasterizer = ref-style stand-in; no optimizer step"}
-        sys.modules["diff_gaussian_rasterization"] = ours
-        importlib.reload(rgr)
-    except Exception as e:  # pragma: no cover
-        out["expansion_error"] = repr(e)
-
-    # (4) image sink vs torchvision.utils.save_image (scripts/render_time_animated.py:86-87), frames per second incl. the files
+    # (2) image sink vs torchvision.utils.save_image (scripts/render_time_animated.py:86-87), frames per second incl. the files
     try:
         import shutil
         import tempfile
@@ -584,7 +535,14 @@ def main():
     ap.add_argument("--reference-ops", action="store_true",
                     help="glue ops as the reference orders them (two-step expansion, ATen loss, torch Adam) around our rasterizer")
     ap.add_argument("--cpu-budget", type=float, default=15.0, help="(kept for compatibility; the CPU sample is now a fixed tile stride)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32; rows of a large "
+                         "array sampled with a fixed seed; at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -658,9 +616,11 @@ def main():
 
     n_frames = []
 
+    last = {}
+
     def step_resident(s):
         ci = shard_cameras(len(cams), s, rank, world)
-        trainer.step(cams_dev[ci], gts[ci])
+        last["loss"] = trainer.step(cams_dev[ci], gts[ci])
         n_frames.append(rasterizer.last_num_rendered)
 
     # e2e: every step's inputs (ground-truth image + 35 camera floats) come from PINNED HOST memory; the copy of step s+1
@@ -722,6 +682,10 @@ def main():
     if sampler:
         sampler.active = False
     launches = _lib.launch_count(reset=True)
+    if rank == 0 and args.dump_outputs:
+        # what the caller of a training step receives: the loss and the updated parameters (Adam consumes the gradients)
+        dump_outputs(args.dump_outputs, {"loss": last["loss"], "vertices": model.vertices, "_alpha": model._alpha, "_scale": model._scale,
+                                         "_opacity": model._opacity, "features": model.get_features})
 
     def run_e2e(u8):
         e2e_mode["u8"] = u8

@@ -1,231 +1,249 @@
-"""-m gpu: the REFERENCE's own, unmodified Python running on the GPU on top of the drop-in module.
+"""-m gpu: the drop-in module and the fused expansion on the GPU against what the REFERENCE's own, unmodified Python computes.
 
-`baseline/_ref` is a verbatim snapshot of the reference's packages made by build() in the build container (git-ignored;
-it travels to the GPU box like the built .so files).  These tests import from it
-  * games.mesh_splatting.scene.gaussian_mesh_model.GaussianMeshModel  (create_from_pcd, update_alpha, prepare_scaling_rot)
-  * renderer.gaussian_renderer.render                                 (renderer/gaussian_renderer/__init__.py:25-111)
-  * renderer.gaussian_animated_renderer.render                        (renderer/gaussian_animated_renderer/__init__.py:21-121)
-  * scene.cameras.MiniCam
-with `diff_gaussian_rasterization` resolving to this repo's shim, and compare image + gradients with the oracle chain
-(oracle/expansion.py -> oracle/gms_oracle.c).  The stock model is used as shipped (its PyTorch expansion on the GPU) and
-again after expansion.patch_mesh_model() swapped the fused kernels in."""
-import math
+tests/golden/make_reference_render_golden.py ran the reference's code on the CPU and stored in tests/golden/reference_*.npz
+  * the raster settings and Gaussians that renderer.gaussian_renderer.render (renderer/gaussian_renderer/__init__.py:25-111)
+    and renderer.gaussian_animated_renderer.render (:21-121) hand the rasterizer for a stock GaussianMeshModel
+    (create_from_pcd, update_alpha, prepare_scaling_rot),
+  * the gradients of the raw parameters its autograd returns when fed the rasterizer gradients of the CPU oracle,
+  * the stock update_alpha / prepare_scaling_rot values,
+  * which PLY property GaussianModel._load_ply puts at each tensor position, and the model_params.pt keys load_ply reads.
+Here the same inputs go through `diff_gaussian_rasterization` (this repo's shim) on the GPU, with the Gaussians either as the
+stock expansion made them or from the fused kernels swapped into a GaussianMeshModel-like instance by
+expansion.patch_mesh_model(); images and radii are compared with the oracle (oracle/gms_oracle.c) rasterizing the same
+Gaussians, gradients with the reference's.  The fixtures keep a fixed sample of each array's rows (`rows<n>` for a leading dimension n):
+everything is computed on the full scene and compared on those rows."""
+import hashlib
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
+import torch.nn as nn
 
+import diff_gaussian_rasterization as dgr
 from gms_b200 import expansion, scenes
-from helpers import settings_from_camera
 from oracle import expansion as oexp
 from oracle import raster
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "baseline"))
-import ref_snapshot  # noqa: E402
-
 pytestmark = pytest.mark.gpu
 
-PIPE = types.SimpleNamespace(debug=False, antialiasing=False, compute_cov3D_python=False, convert_SHs_python=False)
+GRAD_TOL = {"vertices": 5e-3, "_scale": 5e-3, "_alpha": 1e-3}     # through the near-singular 2D covariance (DESIGN.md 2.2)
+SETTINGS = ("image_height", "image_width", "tanfovx", "tanfovy", "bg", "scale_modifier", "viewmatrix", "projmatrix", "sh_degree",
+            "campos", "prefiltered", "debug", "antialiasing")
 
 
-@pytest.fixture(scope="module")
-def ref():
-    import diff_gaussian_rasterization as shim
-    if not ref_snapshot.import_reference(shim):
-        pytest.skip("reference snapshot (baseline/_ref) not present: run __graft_entry__.build() where /root/reference exists")
-    from games.mesh_splatting.scene.gaussian_mesh_model import GaussianMeshModel
-    from games.mesh_splatting.utils.graphics_utils import MeshPointCloud
-    import renderer.gaussian_renderer as r_static
-    import renderer.gaussian_animated_renderer as r_anim
-    from scene.cameras import MiniCam
-    assert r_static.GaussianRasterizer is shim.GaussianRasterizer
-    return types.SimpleNamespace(GaussianMeshModel=GaussianMeshModel, MeshPointCloud=MeshPointCloud, render=r_static.render,
-                                 render_animated=r_anim.render, MiniCam=MiniCam)
+def _golden(golden_dir, name, p):
+    """The stored reference outputs, after checking that they were made from the same raw parameters as `p`."""
+    z = dict(np.load(os.path.join(golden_dir, name)))
+    for k in ("vertices", "faces", "_alpha", "_scale", "_opacity"):
+        assert hashlib.sha256(getattr(p, k).numpy().tobytes()).hexdigest() == str(z["digest" + k]), k
+    return z
 
 
-def _reference_model(ref, p):
-    """A stock GaussianMeshModel built through its own create_from_pcd (gaussian_mesh_model.py:49-84), then given the
-    trained-like appearance of `p` (create_from_pcd starts every opacity at 0.1 and every SH rest coefficient at 0)."""
-    F, K = p._alpha.shape[:2]
-    verts, faces = p.vertices, p.faces
-    tri = verts[faces]
-    alpha_n = torch.relu(p._alpha) + 1e-8
-    alpha_n = alpha_n / alpha_n.sum(-1, keepdim=True)
-    pts = torch.matmul(alpha_n, tri).reshape(-1, 3)
-    pcd = ref.MeshPointCloud(alpha=p._alpha.clone(), points=pts, colors=np.full((F * K, 3), 0.5, np.float32), normals=np.zeros((F * K, 3), np.float32),
-                             vertices=verts.clone(), faces=faces.numpy(), transform_vertices_function=None, triangles=tri.cuda())
-    m = ref.GaussianMeshModel(3)
-    m.create_from_pcd(pcd, 1.0)
-    with torch.no_grad():
-        m._opacity.copy_(p._opacity.cuda()); m._features_dc.copy_(p._features_dc.cuda()); m._features_rest.copy_(p._features_rest.cuda())
-        m._scale.copy_(p._scale.cuda())
-    m.active_sh_degree = 3
-    m.update_alpha(); m.prepare_scaling_rot()
-    return m
+def _rows(z, x):
+    """The rows of `x` (a tensor or array over the full scene) that the fixtures keep."""
+    x = x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
+    return x[z[f"rows{x.shape[0]}"]]
 
 
-def _minicam(ref, cam):
-    return ref.MiniCam(cam.image_width, cam.image_height, cam.FoVy, cam.FoVx, scenes.ZNEAR, scenes.ZFAR,
-                       cam.world_view_transform.cuda(), cam.full_proj_transform.cuda())
+def _settings(z):
+    """The settings render() built (tanfov from the camera's FoV, campos from MiniCam's inverse view matrix)."""
+    v = {k: z[k] for k in SETTINGS}
+    S = raster.Settings(int(v["image_height"]), int(v["image_width"]), float(v["tanfovx"]), float(v["tanfovy"]), v["bg"],
+                        float(v["scale_modifier"]), v["viewmatrix"], v["projmatrix"], int(v["sh_degree"]), v["campos"],
+                        bool(v["prefiltered"]), bool(v["debug"]), bool(v["antialiasing"]))
+    t = lambda a: torch.tensor(a, device="cuda")
+    rs = dgr.GaussianRasterizationSettings(
+        image_height=S.image_height, image_width=S.image_width, tanfovx=S.tanfovx, tanfovy=S.tanfovy, bg=t(S.bg),
+        scale_modifier=S.scale_modifier, viewmatrix=t(S.viewmatrix), projmatrix=t(S.projmatrix), sh_degree=S.sh_degree,
+        campos=t(S.campos), prefiltered=S.prefiltered, debug=S.debug, antialiasing=S.antialiasing)
+    return S, rs
 
 
-def _oracle_chain(p, S, dC, gpu, triangles=None):
-    """Oracle image and gradients of sum(image * dC) w.r.t. the raw mesh-Gaussian parameters.  `gpu` = the (means3D,
-    scales, rotations) the GPU run handed to the rasterizer: they must agree with the oracle's expansion to fp32 rounding
-    and are what the oracle rasterizes (so that integer outputs can be compared bit for bit); the gradient chain runs
-    through the oracle's own expansion graph."""
-    tv, ta, ts = (x.clone().requires_grad_(True) for x in (p.vertices, p._alpha, p._scale))
-    if triangles is None:
-        xyz, sl, rr, _, _ = oexp.expand(tv, p.faces, ta, ts)
-    else:
-        alpha, _, _ = oexp.update_alpha(ta, tv, p.faces)
-        xyz = torch.matmul(alpha, triangles).reshape(-1, 3)
-        sl, rr = oexp.prepare_scaling_rot(triangles, ts, ta.shape[1])
-    top = p._opacity.clone().requires_grad_(True)
-    sc, rot, op, fe = oexp.activate(sl, rr, top, p._features_dc, p._features_rest)
-    gx, gs, gr = (t.detach().cpu() for t in gpu)
-    assert float((gx - xyz.detach()).abs().max()) <= 2e-6 and float((gr - rot.detach()).abs().max()) <= 4e-6
-    assert float(((gs - sc.detach()).abs() / sc.detach()).max()) <= 1e-5
-    st = raster.forward(S, gx, op.detach(), shs=fe.contiguous(), scales=gs, rotations=gr)
-    g = raster.backward(st, dC)
-    outs = [(xyz, g["dL_dmeans3D"]), (sc, g["dL_dscales"]), (rot, g["dL_drotations"]), (op, g["dL_dopacity"])]
-    outs = [(t, torch.tensor(gr).reshape(t.shape)) for t, gr in outs if t.requires_grad]     # animated path: rotation is a constant of the triangles
-    torch.autograd.backward([t for t, _ in outs], [gr for _, gr in outs])
-    grads = dict(vertices=tv.grad, _alpha=ta.grad, _scale=ts.grad, _opacity=top.grad,
-                 _features_dc=torch.tensor(g["dL_dsh"][:, :1]), _features_rest=torch.tensor(g["dL_dsh"][:, 1:]))
-    return st, grads
+class _MeshModel:
+    """The attributes and getters of a GaussianMeshModel instance (scene/gaussian_model.py:95-115) that the renderers use;
+    expansion.patch_mesh_model() supplies update_alpha / prepare_scaling_rot."""
+
+    def __init__(self, p):
+        mk = lambda t: nn.Parameter(t.cuda().float().contiguous().requires_grad_(True))
+        self.vertices, self._alpha, self._scale, self._opacity = (mk(t) for t in (p.vertices, p._alpha, p._scale, p._opacity))
+        self._features_dc, self._features_rest = mk(p._features_dc), mk(p._features_rest)
+        self.faces = p.faces.cuda()
+        self.eps_s0 = 1e-8
+        expansion.patch_mesh_model(self)
+
+    get_xyz = property(lambda self: self._xyz)
+    get_scaling = property(lambda self: torch.exp(self._scaling))
+    get_rotation = property(lambda self: torch.nn.functional.normalize(self._rotation))
+    get_opacity = property(lambda self: torch.sigmoid(self._opacity))
+    get_features = property(lambda self: torch.cat((self._features_dc, self._features_rest), dim=1))
 
 
-def _check_against_oracle(pkg, model, st, ograds, tag, grad_tol):
-    img = pkg["render"].detach().cpu().numpy()
+def _dC(seed, S):
+    rs = np.random.RandomState(seed)
+    return (rs.randn(3, S.image_height, S.image_width) / (S.image_width * S.image_height)).astype(np.float32)
+
+
+def _render(rs, means3D, scales, rotations, opacities, shs, dC):
+    """The rasterizer call of render() (:94-102), then backward of sum(image * dC)."""
+    means2D = torch.zeros_like(means3D, requires_grad=True)
+    img, radii, _ = dgr.GaussianRasterizer(raster_settings=rs)(means3D=means3D, means2D=means2D, shs=shs, colors_precomp=None,
+                                                               opacities=opacities, scales=scales, rotations=rotations,
+                                                               cov3D_precomp=None)
+    (img * torch.tensor(dC, device="cuda")).sum().backward()
+    assert means2D.grad is not None and (radii > 0).dtype == torch.bool
+    return img, radii
+
+
+def _check_against_oracle(img, radii, S, gauss, tag):
+    """Image and radii against the oracle rasterizing the Gaussians the GPU run rasterized."""
+    xyz, sc, rot, op, shs = (t.detach().cpu() for t in gauss)
+    st = raster.forward(S, xyz, op, shs=shs.contiguous(), scales=sc, rotations=rot)
     ok = st.ambiguous == 0
     nb = int((~ok).sum())
-    err = float(np.abs(img - st.color)[:, ok].max())
+    err = float(np.abs(img.detach().cpu().numpy() - st.color)[:, ok].max())
     print(f"[{tag}] P={st.radii.shape[0]} N={st.N} threshold-ambiguous pixels={nb} max|image-oracle| (others)={err:.2e}")
-    np.testing.assert_array_equal(pkg["radii"].cpu().numpy(), st.radii)
+    np.testing.assert_array_equal(radii.cpu().numpy(), st.radii)
     assert err <= 1e-5, err
     assert nb <= 1e-3 * ok.size
-    for k, ref_g in ograds.items():
-        got = getattr(model, k).grad
-        assert got is not None, k
-        scale = max(float(ref_g.abs().max()), 1e-20)
-        e = float((got.detach().cpu().reshape(ref_g.shape) - ref_g).abs().max()) / scale
-        print(f"[{tag}] grad {k}: max err / max|ref| = {e:.2e}")
-        assert e <= grad_tol.get(k, 2e-4), (k, e)
+    return st
 
 
-GRAD_TOL = {"vertices": 5e-3, "_scale": 5e-3, "_alpha": 1e-3}     # through the near-singular 2D covariance (DESIGN.md 2.2)
+def _check_gaussians(z, prefix, xyz, sc, rot):
+    """The GPU expansion reproduces the Gaussians the reference's stock expansion handed the rasterizer."""
+    gx, gs, gr = (_rows(z, t) for t in (xyz, sc, rot))
+    assert float(np.abs(gx - z[prefix + "means3D"]).max()) <= 2e-6 and float(np.abs(gr - z[prefix + "rotations"]).max()) <= 4e-6
+    assert float((np.abs(gs - z[prefix + "scales"]) / z[prefix + "scales"]).max()) <= 1e-5
+
+
+def _check_grads(got, z, prefix, tag):
+    for k, g in got.items():
+        ref_g = z[prefix + "grad" + k]
+        assert g is not None, k
+        scale = max(float(np.abs(ref_g).max()), 1e-20)
+        e = float(np.abs(_rows(z, g).reshape(ref_g.shape) - ref_g).max()) / scale
+        print(f"[{tag}] grad {k}: max err / max|reference| = {e:.2e}")
+        assert e <= GRAD_TOL.get(k, 2e-4), (k, e)
+
+
+def _check_sh_grads(st, dC, m, tag):
+    """Colour gradients pass the reference's get_features unchanged: compare with the oracle's dL/dsh."""
+    g = raster.backward(st, dC)["dL_dsh"]
+    for k, ref_g in (("_features_dc", g[:, :1]), ("_features_rest", g[:, 1:])):
+        ref_g = torch.tensor(ref_g)
+        e = float((getattr(m, k).grad.detach().cpu() - ref_g).abs().max()) / max(float(ref_g.abs().max()), 1e-20)
+        print(f"[{tag}] grad {k}: max err / max|oracle| = {e:.2e}")
+        assert e <= 2e-4, (k, e)
 
 
 @pytest.mark.parametrize("patched", [False, True])
-def test_reference_render_on_stock_mesh_model_matches_oracle(ref, patched):
+def test_reference_render_on_stock_mesh_model_matches_oracle(golden_dir, patched):
     p = scenes.init_mesh_gaussians(*scenes.icosphere(3), K=3, seed=11, trained_like=True)
-    cam = scenes.look_at_camera((2.3, 0.9, 1.1), (0, 0, 0), 400, 304)
-    m = _reference_model(ref, p)
+    z = _golden(golden_dir, "reference_render_static.npz", p)
+    S, rs = _settings(z)
+    dC = _dC(3, S)
+    m = _MeshModel(p)
+    tag = f"render/{'patched' if patched else 'stock'}-expansion"
     if patched:
-        expansion.patch_mesh_model(m)
         m.update_alpha(); m.prepare_scaling_rot()      # train.py:154-157
-    bg = torch.ones(3, device="cuda")
-    pkg = ref.render(_minicam(ref, cam), m, PIPE, bg)
-    rs = np.random.RandomState(3)
-    dC = (rs.randn(3, cam.image_height, cam.image_width) / (cam.image_width * cam.image_height)).astype(np.float32)
-    (pkg["render"] * torch.tensor(dC, device="cuda")).sum().backward()
-    assert pkg["viewspace_points"].grad is not None and pkg["visibility_filter"].dtype == torch.bool
-    S = settings_from_camera(cam, bg=(1, 1, 1))
-    st, og = _oracle_chain(p, S, dC, (m.get_xyz, m.get_scaling, m.get_rotation))
-    _check_against_oracle(pkg, m, st, og, f"render/{'patched' if patched else 'stock'}-expansion", GRAD_TOL)
+        gauss = (m.get_xyz, m.get_scaling, m.get_rotation, m.get_opacity)
+        _check_gaussians(z, "", *gauss[:3])
+    else:
+        # the stock expansion's Gaussians: the oracle's restatement of it, which must give the reference's values
+        xyz, sl, rr, _, _ = oexp.expand(p.vertices, p.faces, p._alpha, p._scale)
+        sc, rot, op, _ = oexp.activate(sl, rr, p._opacity, p._features_dc, p._features_rest)
+        _check_gaussians(z, "", xyz, sc, rot)
+        assert float(np.abs(_rows(z, op) - z["opacities"]).max()) <= 1e-7
+        gauss = tuple(t.detach().cuda().requires_grad_(True) for t in (xyz, sc, rot, op))
+    gauss = gauss + (m.get_features,)
+    img, radii = _render(rs, *gauss, dC)
+    st = _check_against_oracle(img, radii, S, gauss, tag)
+    _check_sh_grads(st, dC, m, tag)
+    if patched:
+        got = {k: getattr(m, k).grad for k in ("vertices", "_alpha", "_scale", "_opacity")}
+    else:
+        # the GPU's rasterizer gradients through the oracle's restatement of the stock expansion (tests/test_oracle_golden.py)
+        tv, ta, ts, top = (x.clone().requires_grad_(True) for x in (p.vertices, p._alpha, p._scale, p._opacity))
+        xyz, sl, rr, _, _ = oexp.expand(tv, p.faces, ta, ts)
+        sc, rot, op, _ = oexp.activate(sl, rr, top, p._features_dc, p._features_rest)
+        torch.autograd.backward([xyz, sc, rot, op], [t.grad.cpu() for t in gauss[:4]])
+        got = dict(vertices=tv.grad, _alpha=ta.grad, _scale=ts.grad, _opacity=top.grad)
+    _check_grads(got, z, "", tag)
 
 
-def test_patched_and_stock_expansion_agree_on_the_gpu(ref):
+def test_patched_and_stock_expansion_agree_on_the_gpu(golden_dir):
     p = scenes.init_mesh_gaussians(*scenes.icosphere(3), K=5, seed=12, trained_like=True)
-    a = _reference_model(ref, p)
-    b = expansion.patch_mesh_model(_reference_model(ref, p))
+    z = _golden(golden_dir, "reference_expansion_k5.npz", p)
+    b = _MeshModel(p)
     b.update_alpha(); b.prepare_scaling_rot()
     for k, tol in (("alpha", 1e-6), ("triangles", 0.0), ("_xyz", 1e-6), ("_scaling", 1e-5), ("_rotation", 2e-6)):
-        x, y = getattr(a, k).detach(), getattr(b, k).detach()
-        assert x.shape == y.shape and float((x - y).abs().max()) <= tol, k
+        x, y = z[k], _rows(z, getattr(b, k))
+        assert x.shape == y.shape and float(np.abs(x - y).max()) <= tol, k
     # alpha stays differentiable on the patched model (renderer/gaussian_animated_renderer/__init__.py:61-64 consumes it)
-    g = torch.randn_like(b.alpha)
-    (b.alpha * g).sum().backward()
-    (a.alpha * g).sum().backward()
-    assert float((a._alpha.grad - b._alpha.grad).abs().max()) <= 1e-5 * float(a._alpha.grad.abs().max())
+    g = np.random.RandomState(12).randn(*b.alpha.shape).astype(np.float32)
+    (b.alpha * torch.tensor(g, device="cuda")).sum().backward()
+    ref_g = z["grad_alpha"]
+    assert float(np.abs(_rows(z, b._alpha.grad) - ref_g).max()) <= 1e-5 * float(np.abs(ref_g).max())
 
 
 @pytest.mark.parametrize("t", [0.0, 2.1, 5.7])
-def test_reference_animated_renderer_matches_oracle(ref, t):
+def test_reference_animated_renderer_matches_oracle(golden_dir, t):
     """scripts/render_time_animated.py:68-87: vertices moved by transform_hotdog_fly(t), triangles gathered, and
     gaussian_animated_renderer.render(idxs, triangles, ...) re-expanding from them -- here with gradients as well."""
     p = scenes.init_mesh_gaussians(*scenes.icosphere(3), K=3, seed=13, trained_like=True)
-    cam = scenes.look_at_camera((2.6, -0.7, 0.8), (0, 0, 0), 368, 272)
-    m = expansion.patch_mesh_model(_reference_model(ref, p))
+    z = _golden(golden_dir, "reference_render_animated.npz", p)
+    i = [float(x) for x in z["times"]].index(t)
+    S, rs = _settings(z)
+    m = _MeshModel(p)
     m.update_alpha(); m.prepare_scaling_rot()
-    new_v = scenes.transform_hotdog_fly(p.vertices, t)
-    tri = new_v[p.faces]
-    bg = torch.ones(3, device="cuda")
-    pkg = ref.render_animated(None, tri.cuda(), _minicam(ref, cam), m, PIPE, bg)
-    rs = np.random.RandomState(4)
-    dC = (rs.randn(3, cam.image_height, cam.image_width) / (cam.image_width * cam.image_height)).astype(np.float32)
-    (pkg["render"] * torch.tensor(dC, device="cuda")).sum().backward()
-    S = settings_from_camera(cam, bg=(1, 1, 1))
-    with torch.no_grad():
-        means3D = torch.matmul(m.alpha, tri.cuda()).reshape(-1, 3)     # the renderer's own expression (:61-67)
-    st, og = _oracle_chain(p, S, dC, (means3D, m.get_scaling, m.get_rotation), triangles=tri)
-    og.pop("vertices")                      # the animated path feeds triangles directly: no gradient reaches pc.vertices
-    _check_against_oracle(pkg, m, st, og, f"animated t={t}", GRAD_TOL)
+    tri = scenes.transform_hotdog_fly(p.vertices, t)[p.faces].cuda()
+    # what the animated renderer does with the triangles (:61-73)
+    means3D = torch.matmul(m.alpha, tri).reshape(-1, 3)
+    m.triangles = tri
+    m.prepare_scaling_rot()
+    gauss = (means3D, m.get_scaling, m.get_rotation, m.get_opacity)
+    _check_gaussians(z, f"t{i}_", *gauss[:3])
+    gauss = gauss + (m.get_features,)
+    dC = _dC(4, S)
+    img, radii = _render(rs, *gauss, dC)
+    st = _check_against_oracle(img, radii, S, gauss, f"animated t={t}")
+    _check_sh_grads(st, dC, m, f"animated t={t}")
+    _check_grads({k: getattr(m, k).grad for k in ("_alpha", "_scale", "_opacity")}, z, f"t{i}_", f"animated t={t}")
+    # the animated path feeds triangles directly: no gradient reaches pc.vertices
+    assert m.vertices.grad is None or not m.vertices.grad.any()
 
 
-def test_checkpoint_written_here_loads_in_the_reference(ref, tmp_path):
-    """io_ply.save_mesh_model -> the reference's own GaussianMeshModel.load_ply (gaussian_mesh_model.py:211-225 ->
-    scene/gaussian_model.py:226-262) -> its render(): the same image as the model that was saved.  `plyfile` is absent from
-    the image; the reference's loader is served by a reader that implements the three things it uses
-    (PlyData.read, elements[0][name], elements[0].properties[i].name) on top of the PLY specification."""
-    import sys
-    import types as _t
+def test_checkpoint_written_here_loads_in_the_reference(golden_dir, tmp_path):
+    """io_ply.save_mesh_model -> the tensors the reference's GaussianMeshModel.load_ply (gaussian_mesh_model.py:211-225 ->
+    scene/gaussian_model.py:226-262) builds from it, assembled with the property layout its loader was seen to use ->
+    the same image as the model that was saved."""
     from gms_b200 import io_ply
     from gms_b200.model import MeshGaussianModel
     from gms_b200.trainer import render_frame
-
-    class _El:
-        def __init__(self, data, names):
-            self.data, self.properties = data, [_t.SimpleNamespace(name=n) for n in names]
-
-        def __getitem__(self, k):
-            return self.data[k]
-
-    class _PlyData:
-        def __init__(self, elements):
-            self.elements = elements
-
-        @staticmethod
-        def read(path):
-            data, names = io_ply.read_ply_vertices(path)
-            return _PlyData([_El(data, names)])
-
-    import scene.gaussian_model as sgm
-    old = sgm.PlyData
-    sgm.PlyData = _PlyData
-    try:
-        p = scenes.init_mesh_gaussians(*scenes.icosphere(3), K=3, seed=31, trained_like=True)
-        ours = MeshGaussianModel.from_params(p, "cuda")
-        ply = str(tmp_path / "point_cloud" / "iteration_30000" / "point_cloud.ply")
-        io_ply.save_mesh_model(ply, ours)
-        m = ref.GaussianMeshModel(3)
-        m.load_ply(ply)
-        m.active_sh_degree = 3
-        assert m.vertices.is_cuda and m._alpha.is_cuda and m.faces.is_cuda          # used where they are: no .cuda() in the reference
-        m.update_alpha(); m.prepare_scaling_rot()
-        cam = scenes.look_at_camera((2.3, 0.9, 1.1), (0, 0, 0), 320, 240)
-        bg = torch.ones(3, device="cuda")
-        with torch.no_grad():
-            a = ref.render(_minicam(ref, cam), m, PIPE, bg)["render"]
-            b = render_frame(ours, cam.to("cuda"), bg, fused=False)[0]
-        # the reference's PyTorch expansion and the fused kernels agree to ~1e-7 on the Gaussians, so the two images agree to
-        # 1e-5 except where a 1/255 blending threshold flips (a handful of pixels, each by at most one splat's contribution)
-        err = (a - b).abs().amax(dim=0)
-        assert float((err > 1e-5).float().mean()) <= 1e-3 and float(err.max()) <= 2e-2, (float((err > 1e-5).float().mean()), float(err.max()))
-    finally:
-        sgm.PlyData = old
+    lay = np.load(os.path.join(golden_dir, "reference_ply_layout.npz"))
+    p = scenes.init_mesh_gaussians(*scenes.icosphere(3), K=3, seed=31, trained_like=True)
+    ours = MeshGaussianModel.from_params(p, "cuda")
+    ply = str(tmp_path / "point_cloud" / "iteration_30000" / "point_cloud.ply")
+    io_ply.save_mesh_model(ply, ours)
+    data, names = io_ply.read_ply_vertices(ply)
+    loaded = {}
+    for k in ("_xyz", "_features_dc", "_features_rest", "_opacity", "_scaling", "_rotation"):
+        props = lay["property_names"][lay[k]]
+        assert all(n in names for n in props.ravel()), (k, props)
+        loaded[k] = torch.tensor(np.stack([np.asarray(data[n], np.float32) for n in props.ravel()], -1).reshape(len(data), *props.shape))
+    params = torch.load(ply.replace("point_cloud.ply", "model_params.pt"))
+    for k in lay["model_params_keys"]:
+        assert k in params, k
+    assert params["vertices"].is_cuda and params["_alpha"].is_cuda and params["faces"].is_cuda   # used where they are: no .cuda() in the reference
+    d = lambda t: t.detach().cpu()
+    q = scenes.MeshGaussianParams(d(params["vertices"]), d(params["faces"]), d(params["_alpha"]), d(params["_scale"]),
+                                  loaded["_features_dc"], loaded["_features_rest"], loaded["_opacity"])
+    m = MeshGaussianModel.from_params(q, "cuda")
+    cam = scenes.look_at_camera((2.3, 0.9, 1.1), (0, 0, 0), 320, 240)
+    bg = torch.ones(3, device="cuda")
+    with torch.no_grad():
+        a = render_frame(m, cam.to("cuda"), bg, fused=False)[0]
+        b = render_frame(ours, cam.to("cuda"), bg, fused=False)[0]
+    # a 1/255 blending threshold may flip on a handful of pixels, each by at most one splat's contribution
+    err = (a - b).abs().amax(dim=0)
+    assert float((err > 1e-5).float().mean()) <= 1e-3 and float(err.max()) <= 2e-2, (float((err > 1e-5).float().mean()), float(err.max()))
